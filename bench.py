@@ -22,6 +22,8 @@ A "step" is one pass of the hot path over one batch of synthetic input:
     `create_proof_k14_real` (a real proof of the reference's benchmark circuit through the engine's API, verified through the engine).
 
 `--impl reference` times that CPU restatement alone (the reference arm).
+`--dump-outputs DIR` writes what the last timed step computed, from inputs that are the same on every run, so that two builds
+can be compared output for output.
 """
 import argparse
 import ctypes
@@ -99,6 +101,14 @@ class ClockSampler:
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each named array of 32-byte canonical field elements as out_dir/<name>.npy: float64, one column per
+    little-endian 32-bit limb (float64 holds every limb exactly, so two runs compare bit for bit)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.uint8).view("<u4").astype(np.float64))
+
+
 def rand_canonical_scalars(torch, n, seed, device):
     """n uniform-ish canonical scalars (< 2^254 < modulus) as an (n, 8) int32 tensor."""
     g = torch.Generator(device=device).manual_seed(seed)
@@ -122,8 +132,10 @@ def run_reference(args, rank, world):
         cref.best_multiexp(CURVE, kb, pb, threads)
     t0 = time.time()
     for _ in range(args.steps):
-        cref.best_multiexp(CURVE, kb, pb, threads)
-    dt = (time.time() - t0) / max(args.steps, 1)
+        got = cref.best_multiexp(CURVE, kb, pb, threads)
+    dt = (time.time() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"msm": got.reshape(2, 32)})
     value = n / dt
     sample = f"{args.steps} x full 2^{LOG_N}-pair best_multiexp (window-parallel, c=ceil(ln n)=14, 19 window tasks)"
     line = {
@@ -727,7 +739,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy: msm (the affine x, y of "
+                         "the MSM result) and, for the ours arm, ntt_fp / ntt_fq (a fixed sample of the transforms' outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -812,6 +829,9 @@ def main():
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop(t_wall0, t_wall1)
     launches = L.launch_count() - launches0
+    dumps = {}
+    if args.dump_outputs and rank == 0:
+        dumps["msm"] = result_affine().reshape(2, 32)
     if world > 1:
         t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -992,6 +1012,14 @@ def main():
         e1.record(stream)
         torch.cuda.synchronize()
         ntt_ms = e0.elapsed_time(e1) / args.steps
+
+        def ntt_sample(field, out):
+            """4096 fixed positions of a transform's output (256 KiB instead of 32 MiB), Montgomery -> canonical."""
+            s = out[torch.randperm(n, generator=torch.Generator().manual_seed(SEED))[:4096].sort().values.to(dev)]
+            L.check(lib.h2_dev_convert(L.FIELD_ID[field], ctypes.c_void_p(s.data_ptr()), ctypes.c_size_t(s.shape[0]), 0, sp))
+            return s.cpu().numpy().view(np.uint8)
+        if args.dump_outputs:
+            dumps["ntt_fp"] = ntt_sample("fp", outs[(args.steps - 1) % 5])
         L.check(lib.h2_profile_enable(1))
         for i in range(5):
             ntt_step(i)
@@ -1044,6 +1072,8 @@ def main():
         e1.record(stream)
         torch.cuda.synchronize()
         nttq_ms = e0.elapsed_time(e1) / args.steps
+        if args.dump_outputs:
+            dumps["ntt_fq"] = ntt_sample("fq", outs[(args.steps - 1) % 5])
         extra["ntt_fq"] = {"metric": "ntt_elems_per_s", "value": n / (nttq_ms * 1e-3), "unit": "elems/s", "ms_per_step": nttq_ms,
                            "config": {"workload": f"best_fft 2^{LOG_N} over Fq (configs[1] as written: the Vesta scalar field)"}}
         del qbufs, aq
@@ -1124,6 +1154,8 @@ def main():
             "multi_gpu_parity": parity_multi, "extra": extra,
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumps)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
